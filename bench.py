@@ -248,7 +248,7 @@ class Token:
                 y2 = torch.empty((2, 1, a["n"]), dtype=a["y"].dtype, device=dev)
                 xh2 = torch.empty((2, 1, a["k"]), dtype=torch.half, device=dev)
                 out.append(dict(kind="mgemm", x=a["x"].view(1, 1, -1), y=y2, xh=xh2, K=a["K"], reduce=False,
-                                B=ptr("tr"), suh=ptr("suh"), svh=ptr("svh"), snl=None, cp=None, shared_inputs=2))
+                                B=ptr("tr"), suh=ptr("suh"), svh=ptr("svh"), snl=None, cp=None, shared_inputs=2, mats=(a, b)))
                 i += 2
             else:
                 out.append(dict(kind="gemm", mt=a, reduce=a["reduce"]))
@@ -262,6 +262,20 @@ class Token:
             if ln["kind"] == "mgemm":
                 b -= 2 * ln["x"].shape[-1] * (ln["shared_inputs"] - 1)
         return b
+
+    def outputs(self):
+        """What the caller of the timed launch list receives after a step: every projection's output as float32, stacked
+        over layers ({"q": (layers, 1, n), ..., "lm_head": (1, 1, vocab)}).  A two-matrix exl3_mgemm writes its own (2, 1, n)
+        output; every other launch writes the matrix's y."""
+        out_of = {id(mt): mt["y"] for mt in self.mats}
+        if self.mode == "ops":
+            for ln in self.launches:
+                for j, mt in enumerate(ln.get("mats", ())):
+                    out_of[id(mt)] = ln["y"][j]
+        by_name = {}
+        for mt in self.mats:
+            by_name.setdefault(mt["name"], []).append(out_of[id(mt)])
+        return {name: self.torch.stack(ys).float().cpu().numpy() for name, ys in by_name.items()}
 
     def build_chains(self, mode):
         """
@@ -535,6 +549,15 @@ def ncu_traffic_per_launch(tok):
         return None
 
 
+def dump_outputs(tok, out_dir):
+    """The outputs of the last timed step as out_dir/<projection>.npy (float32; Llama-3.1-8B: 6.0 MB, 70B: 27.4 MB).  The inputs
+    come from the seeded generator of Token, so two builds run with the same arguments can be compared output for output."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in tok.outputs().items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def run_gpu_arm(args, cfg):
     import torch
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -626,6 +649,8 @@ def run_gpu_arm(args, cfg):
     ms = timed(step, args.steps)
     clocks = sampler.stop() if rank == 0 else None
     ms_per_step = ms / args.steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(tok, args.dump_outputs)
 
     # ---- the same token with the reference's Llama launch list (q, k+v as two calls), same run, same weights ----
     ref_list = None
@@ -783,7 +808,10 @@ def main():
                          "exl3_gemm_allreduce")
     ap.add_argument("--tp-shapes", type=int, default=0, help="debug: run rank 0's shard shapes of a TP-N token on one GPU without the all-reduce")
     ap.add_argument("--cpu-budget", type=float, default=0.0, help="seconds; 0 = the fixed sample (all of layer 0)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write rank 0's outputs of the last timed step to DIR/<projection>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     cfg = MODELS[args.model]
     if args.impl == "reference":
         run_reference_arm(args, cfg)

@@ -157,3 +157,30 @@ def test_ncu_capture_parser_is_unit_aware(tmp_path):
     f = tmp_path / "cap.csv"
     f.write_text("metric,unit,value\ndram__bytes_read.sum,Gbyte,1.5\ndram__bytes_write.sum,Kbyte,2\n")
     assert bench.ncu_dram_bytes(str(f)) == 1.5e9 + 2e3
+
+
+@pytest.mark.parametrize("fanout", [True, False])
+def test_dumped_outputs_are_what_each_launch_wrote(fanout, tmp_path):
+    """--dump-outputs: every projection's output as float32, stacked over layers, taken from the buffer its launch writes
+    (a two-matrix exl3_mgemm's own output, otherwise the matrix's y); within 64 MB for both bench models."""
+    import numpy as np
+    tok = bench.Token(TINY, 1, 0, torch.device("cpu"), fanout=fanout)
+    for i, mt in enumerate(tok.mats):
+        mt["y"].fill_(i)
+    pair = {}
+    for ln in tok.launches:
+        for j, mt in enumerate(ln.get("mats", ())):
+            i = next(i for i, t in enumerate(tok.mats) if t is mt)
+            ln["y"][j].fill_(1000 + i); pair[i] = True
+    names = ["q", "k", "v", "o", "gate", "up", "down"]
+    assert {tok.mats[i]["name"] for i in pair} == ({"gate", "up"} if fanout else {"k", "v", "gate", "up"})
+    bench.dump_outputs(tok, str(tmp_path))
+    assert sorted(p.name for p in tmp_path.iterdir()) == sorted(f"{n}.npy" for n in names + ["lm_head"])
+    for name in names + ["lm_head"]:
+        a = np.load(tmp_path / f"{name}.npy")
+        idx = [i for i, t in enumerate(tok.mats) if t["name"] == name]
+        assert a.dtype == np.float32 and a.shape == (len(idx), 1, tok.mats[idx[0]]["n"])
+        assert [float(v) for v in a[:, 0, 0]] == [1000.0 + i if i in pair else float(i) for i in idx]
+    for cfg in bench.MODELS.values():
+        layer, head = bench.token_plan(cfg, 1)
+        assert 4 * (cfg["layers"] * sum(n for (_, _, n, _, _, _) in layer) + head[2]) <= 64 << 20

@@ -1,70 +1,27 @@
 """
-Drop-in check at the Python level, run where the reference checkout exists (this container; skipped on the GPU box): the
-REFERENCE'S OWN `exllamav3/modules/quant/exl3.py` (LinearEXL3) is loaded from /root/reference -- unmodified, never copied --
-with its `ext` import bound to this repo's shim (`exllamav3_b200.ext`), exactly what INTEGRATION.md's three-line patch does.
-Every call the reference module then makes into the extension is bound against the shim's real signatures (a wrong argument
-count or a missing name fails here), and the reference's dispatch is compared with this repo's own minimal caller (QLinear)
-on the same inputs: both must issue the same extension calls with the same argument shapes.  No kernel runs: the shim's entry points are wrapped by recorders after their signatures have been checked.
+Drop-in check at the Python level against the REFERENCE'S OWN modules (`exllamav3/modules/quant/exl3.py` LinearEXL3,
+`modules/multilinear.py`, `model/config.py`): oracle/gen_golden_callsites.py ran them unmodified with their `ext` import bound
+to this repo's shim (`exllamav3_b200.ext`), exactly what INTEGRATION.md's three-line patch does, and recorded every extension
+call they made (bound against the shim's real signatures) in tests/golden/ref_callsites.json.  Here this repo's own minimal
+caller (QLinear, pointer_tables, tp.tp_slice) runs on the same inputs and must issue the same extension calls with the same
+argument shapes, and every recorded call must still fit the shim's signatures.  No kernel runs: the shim's entry points are
+wrapped by recorders after their signatures have been checked.
 """
-import importlib.util, inspect, os, sys, types
+import inspect, json, os
 import pytest
 import torch
 
-REF = "/root/reference/exllamav3"
-pytestmark = pytest.mark.skipif(not os.path.isfile(os.path.join(REF, "modules", "quant", "exl3.py")),
-                                reason="reference checkout not present (GPU box)")
+import refstubs
+from conftest import GOLDEN
+
+REF = json.load(open(os.path.join(GOLDEN, "ref_callsites.json")))
+DTYPES = {None: None, "float16": torch.half, "float32": torch.float}
 
 
 @pytest.fixture()
-def ref_exl3(monkeypatch):
+def recorded(monkeypatch):
     from exllamav3_b200 import ext
-    import refstubs
-    calls = []
-
-    def wrap(name):
-        real = getattr(ext, name)
-        sig = inspect.signature(real)
-
-        def f(*a, **kw):
-            sig.bind(*a, **kw)                                    # the reference's argument list fits the shim's signature
-            calls.append((name,) + tuple(tuple(t.shape) if isinstance(t, torch.Tensor) else t for t in a))
-            return 210
-        return f
-
-    for name in ("exl3_gemm", "had_r_128", "reconstruct", "reconstruct_slice", "reconstruct_had_slice", "hgemm"):
-        monkeypatch.setattr(ext, name, wrap(name))
-
-    def mod(name, **attrs):
-        m = types.ModuleType(name)
-        m.__path__ = []
-        for k, v in attrs.items():
-            setattr(m, k, v)
-        monkeypatch.setitem(sys.modules, name, m)
-        return m
-
-    class Config: pass
-    mod("exllamav3")
-    mod("exllamav3.model")
-    mod("exllamav3.model.config", Config=Config, NullConfig=refstubs.NullConfig)
-    mod("exllamav3.ext", exllamav3_ext=ext)                       # <- INTEGRATION.md: the extension module IS the shim
-    mod("exllamav3.util", profile_opt=lambda f: f)
-    mod("exllamav3.util.tensor", g_tensor_cache=refstubs.g_tensor_cache)
-    mod("exllamav3.modules")
-    mod("exllamav3.modules.quant")
-    mod("exllamav3.modules.quant.exl3_lib")
-    mod("exllamav3.modules.quant.exl3_lib.quantize", preapply_had_l=refstubs.preapply_had_l, preapply_had_r=refstubs.preapply_had_r,
-        had_k=128, had_n=128)
-    spec = importlib.util.spec_from_file_location("exllamav3.modules.quant.exl3", os.path.join(REF, "modules", "quant", "exl3.py"))
-    m = importlib.util.module_from_spec(spec)
-    monkeypatch.setitem(sys.modules, "exllamav3.modules.quant.exl3", m)
-    spec.loader.exec_module(m)
-    return m, calls
-
-
-def _tensors(k, n, K=4):
-    g = torch.Generator().manual_seed(1)
-    tr = torch.randint(0, 32767, (k // 16, n // 16, 16 * K), generator=g, dtype=torch.int32).to(torch.int16)
-    return dict(suh=torch.ones(k, dtype=torch.half), svh=torch.ones(n, dtype=torch.half), trellis=tr, mul1=torch.zeros((), dtype=torch.int))
+    return refstubs.install_recorders(ext, monkeypatch.setattr)
 
 
 def _qlin(t, **kw):
@@ -72,98 +29,83 @@ def _qlin(t, **kw):
     return QLinear(t["trellis"], t["suh"], t["svh"], mul1=True, **kw)
 
 
-def test_reference_linear_exl3_runs_on_the_shim_and_matches_the_mirror(ref_exl3):
-    ref_mod, calls = ref_exl3
-    from exllamav3_b200 import qlinear
-    assert ref_mod.AUTO_RECONSTRUCT_THRESHOLD == qlinear.KERNEL_MAX_ROWS == 144
-    assert ref_mod.MAX_RECONSTRUCT_SLICE_N == qlinear.DENSE_WINDOW_COLS == 32768
-    k, n = 256, 384
-    ref_lin = ref_mod.LinearEXL3(None, k, n, key="q", **_tensors(k, n))          # constructs ext.BC_LinearEXL3 from the shim
-    mir_lin = _qlin(_tensors(k, n))
+def _fits_shim(calls):
+    """Every recorded call of the reference still binds against the shim's current signature."""
     from exllamav3_b200 import ext
-    assert isinstance(ref_lin.bc, ext.BC_LinearEXL3) and ref_lin.K == 4 and ref_lin.mul1 and not ref_lin.mcg
-    for (shape, params, out_dtype) in (((1, k), {}, None), ((144, k), {}, torch.float), ((3, 7, k), {}, None),
-                                       ((145, k), {}, None), ((1, k), {"reconstruct": True}, None), ((1024, k), {}, torch.float)):
-        x = torch.zeros(shape, dtype=torch.half)
-        calls.clear(); yr = ref_lin.forward(x, params, out_dtype); seq_ref = list(calls)
-        calls.clear(); ym = mir_lin.forward(x, params, out_dtype); seq_mir = list(calls)
-        assert seq_ref == seq_mir and len(seq_ref) >= 1, (shape, params)            # same extension calls, same argument shapes
-        assert yr.shape == ym.shape == tuple(shape[:-1]) + (n,) and yr.dtype == ym.dtype
+    for c in calls:
+        inspect.signature(getattr(ext, c[0])).bind(*c[1:])
+
+
+def test_reference_linear_exl3_runs_on_the_shim_and_matches_the_mirror(recorded):
+    from exllamav3_b200 import ext, qlinear
+    calls = recorded
+    assert REF["constants"]["AUTO_RECONSTRUCT_THRESHOLD"] == qlinear.KERNEL_MAX_ROWS == 144
+    assert REF["constants"]["MAX_RECONSTRUCT_SLICE_N"] == qlinear.DENSE_WINDOW_COLS == 32768
+    lin = REF["linear"]
+    k, n = lin["k"], lin["n"]
+    # the reference constructs ext.BC_LinearEXL3 from the shim: its arguments bind against the shim's constructor
+    ctor = REF["bc_ctor"]
+    inspect.signature(ext.BC_LinearEXL3).bind(*ctor["args"], **{kw: None for kw in ctor["kwargs"]})
+    t = refstubs.linear_tensors(k, n)
+    assert ctor["args"][:3] == [list(t["trellis"].shape), [k], [n]] and ctor["args"][3:7] == [4, None, False, True]
+    assert isinstance(ext.BC_LinearEXL3(t["trellis"], t["suh"], t["svh"], 4, None, False, True, None), ext.BC_LinearEXL3)
+    assert lin["K"] == 4 and lin["mul1"] and not lin["mcg"]
+    mir_lin = _qlin(t)
+    for case in lin["cases"]:
+        _fits_shim(case["calls"])
+        calls.clear()
+        ym = mir_lin.forward(torch.zeros(case["shape"], dtype=torch.half), case["params"], DTYPES[case["out_dtype"]])
+        seq_mir = refstubs.jsonable(calls)
+        assert case["calls"] == seq_mir and len(seq_mir) >= 1, case      # same extension calls, same argument shapes
+        assert case["y_shape"] == list(ym.shape) == case["shape"][:-1] + [n] and DTYPES[case["y_dtype"]] == ym.dtype
     # the kernel path hands exl3_gemm the reference's 10 arguments: (A, B, C, suh, A_had, svh, -1, mcg, mul1, 0)
-    calls.clear(); ref_lin.forward(torch.zeros((2, k), dtype=torch.half), {})
-    assert calls[0][0] == "exl3_gemm" and calls[0][7:] == (-1, False, True, 0)
+    two_rows = next(c for c in lin["cases"] if c["shape"] == [2, k] and not c["params"])
+    assert two_rows["calls"][0][0] == "exl3_gemm" and two_rows["calls"][0][7:] == [-1, False, True, 0]
 
 
-def test_reference_wide_output_slicing_matches_the_mirror(ref_exl3, monkeypatch):
-    ref_mod, calls = ref_exl3
+def test_reference_wide_output_slicing_matches_the_mirror(recorded, monkeypatch):
     from exllamav3_b200 import qlinear
-    monkeypatch.setattr(ref_mod, "MAX_RECONSTRUCT_SLICE_N", 256)
-    monkeypatch.setattr(qlinear, "DENSE_WINDOW_COLS", 256)
-    k, n = 128, 640
-    ref_lin = ref_mod.LinearEXL3(None, k, n, **_tensors(k, n)); mir_lin = _qlin(_tensors(k, n))
-    for rows in (200, 2048):
-        x = torch.zeros((rows, k), dtype=torch.half)
-        calls.clear(); ref_lin.forward(x, {}); a = list(calls)
-        calls.clear(); mir_lin.forward(x, {}); b = list(calls)
-        assert a == b and sum(c[0] == "hgemm" for c in a) == 3
+    calls = recorded
+    wide = REF["wide"]
+    monkeypatch.setattr(qlinear, "DENSE_WINDOW_COLS", wide["slice_n"])
+    mir_lin = _qlin(refstubs.linear_tensors(wide["k"], wide["n"]))
+    assert [c["rows"] for c in wide["cases"]] == [200, 2048]
+    for case in wide["cases"]:
+        _fits_shim(case["calls"])
+        calls.clear(); mir_lin.forward(torch.zeros((case["rows"], wide["k"]), dtype=torch.half), {})
+        assert case["calls"] == refstubs.jsonable(calls) and sum(c[0] == "hgemm" for c in case["calls"]) == 3
 
 
 def test_reference_multilinear_tables_match_the_mirror():
     """modules/multilinear.py builds the pointer tables exl3_mgemm reads; pointer_tables must build the same ones."""
-    src = open(os.path.join(REF, "modules", "multilinear.py")).read()
-    ns = {}
-    exec(compile(src.replace("from . import Linear", "Linear = object"), "multilinear_ref", "exec"), ns)     # executed in memory, not copied
     from exllamav3_b200 import pointer_tables
-    k, n = 128, 256
-    inners = [_qlin(_tensors(k, n)) for _ in range(3)]
-    for i in inners:
-        i.quant_type = "exl3"                                   # the attribute the reference's table builder asserts on
-
-    class Lin:                                                  # the reference wraps LinearEXL3 in modules.Linear (.inner)
-        def __init__(self, inner):
-            self.inner, self.quant_type, self.softcap, self.post_scale = inner, "exl3", 0.0, 1.0
-            self.in_features, self.out_features = inner.in_features, inner.out_features
-    ref_ml = ns["MultiLinear"]("cpu", [Lin(i) for i in inners])
+    ml_ref = REF["multilinear"]
+    k, n = ml_ref["k"], ml_ref["n"]
+    inners = [_qlin(refstubs.linear_tensors(k, n)) for _ in range(ml_ref["count"])]
+    where = {getattr(i, a).data_ptr(): [a, j] for j, i in enumerate(inners) for a in ("trellis", "suh", "svh")}
     ml = dict(zip(("ptrs_trellis", "ptrs_suh", "ptrs_svh"), pointer_tables("cpu", inners)))
     for a in ("ptrs_trellis", "ptrs_suh", "ptrs_svh"):
-        assert torch.equal(getattr(ref_ml, a), ml[a]) and ml[a].dtype == torch.long
-    assert (ref_ml.K, ref_ml.mcg, ref_ml.mul1, ref_ml.in_features, ref_ml.out_features) == (4, False, True, k, n)
+        assert ml[a].dtype == torch.long and ml_ref["tables"][a]["dtype"] == "int64"
+        assert [where.get(p) for p in ml[a].tolist()] == ml_ref["tables"][a]["entries"]
+    i0 = inners[0]
+    assert (ml_ref["K"], ml_ref["mcg"], ml_ref["mul1"], ml_ref["in_features"], ml_ref["out_features"]) == \
+           (i0.K, i0.mcg, i0.mul1, i0.in_features, i0.out_features) == (4, False, True, k, n)
 
 
 def test_every_reference_call_site_of_the_qgemm_surface_fits_the_shim():
     """Static audit: every `ext.<op>(...)` call in the reference's Python sources, for the ops of the qgemm path, is bound
     (by argument count and keyword names) against the shim's signature.  SURVEY.md 8b lists these callers."""
-    import ast
     from exllamav3_b200 import ext
-    ops = ["exl3_gemm", "exl3_mgemm", "reconstruct", "reconstruct_slice", "reconstruct_had_slice", "had_r_128", "hgemm",
-           "exl3_gemv", "g_get_cc", "g_get_num_sms", "exl3_gemv_int8_max_k", "exl3_gemm_num_kernel_shapes", "exl3_gemm_shape_compat"]
-    sigs = {o: inspect.signature(getattr(ext, o)) for o in ops}
-    seen = {o: 0 for o in ops}
-    files = 0
-    for root, _, names in os.walk(os.path.dirname(REF)):            # the package, science/ (qgemm_benchmark.py), tests/, eval/
-        if "exllamav3_ext" in root:
-            continue
-        for nm in names:
-            if not nm.endswith(".py"):
-                continue
-            path = os.path.join(root, nm)
-            try:
-                tree = ast.parse(open(path).read())
-            except SyntaxError:
-                continue
-            files += 1
-            for node in ast.walk(tree):
-                if (isinstance(node, ast.Call) and isinstance(node.func, ast.Attribute) and node.func.attr in sigs
-                        and isinstance(node.func.value, ast.Name) and node.func.value.id == "ext"):
-                    if any(isinstance(a, ast.Starred) for a in node.args) or any(k.arg is None for k in node.keywords):
-                        continue
-                    op = node.func.attr
-                    try:
-                        sigs[op].bind(*([None] * len(node.args)), **{k.arg: None for k in node.keywords})
-                    except TypeError as e:
-                        raise AssertionError(f"{path}:{node.lineno}: ext.{op} call does not fit the shim: {e}")
-                    seen[op] += 1
-    assert files > 50
+    audit = REF["callsites"]
+    sigs = {o: inspect.signature(getattr(ext, o)) for o in audit["ops"]}
+    seen = {o: 0 for o in audit["ops"]}
+    for s in audit["sites"]:
+        try:
+            sigs[s["op"]].bind(*([None] * s["nargs"]), **{kw: None for kw in s["kwargs"]})
+        except TypeError as e:
+            raise AssertionError(f"{s['path']}:{s['line']}: ext.{s['op']} call does not fit the shim: {e}")
+        seen[s["op"]] += 1
+    assert audit["files"] > 50
     assert seen["exl3_gemm"] >= 1 and seen["exl3_gemm_num_kernel_shapes"] >= 1 and seen["exl3_gemm_shape_compat"] >= 1   # science/qgemm_benchmark.py
     # the call sites SURVEY.md 8b names exist and were checked
     assert seen["exl3_mgemm"] >= 8 and seen["hgemm"] >= 3 and seen["had_r_128"] >= 2 and seen["reconstruct"] >= 2
@@ -175,67 +117,33 @@ def test_reference_use_mgemm_policy_with_the_shims_answer(monkeypatch):
     gate+up stay fused for every bitrate -- the launch list bench.py times (161 launches) -- whereas with the reference
     extension's answer on Blackwell (6) the wide 4-bpw gate+up pair is unfused (225-launch variant, bench.py --no-fuse)."""
     from exllamav3_b200 import ext
-
-    def mod(name, **attrs):
-        m = types.ModuleType(name); m.__path__ = []
-        for k, v in attrs.items():
-            setattr(m, k, v)
-        monkeypatch.setitem(sys.modules, name, m)
-
-    mod("exllamav3"); mod("exllamav3.model"); mod("exllamav3.util")
-    mod("exllamav3.util.rope", RopeSettings=object, RopeStyle=object)
-    mod("exllamav3.loader", SafetensorsCollection=object)
-    mod("exllamav3.util.file", read_dict=None, no_value=None, no_default=None)
-    mod("exllamav3.ext", exllamav3_ext=ext)
-    for v in ("EXL3_INT8_GEMV", "EXL3_MGEMM_K_THRESHOLD", "EXL3_MGEMM_N_THRESHOLD"):
-        monkeypatch.delenv(v, raising=False)
-    spec = importlib.util.spec_from_file_location("exllamav3.model.config", os.path.join(REF, "model", "config.py"))
-    cfg = importlib.util.module_from_spec(spec)
-    monkeypatch.setitem(sys.modules, "exllamav3.model.config", cfg)
-    spec.loader.exec_module(cfg)
-    ip = cfg.InferParams()
     monkeypatch.setattr(ext, "_check", lambda rc: 148)                      # no device here: the index check is not under test
-    assert ext.exl3_gemv_int8_max_k(0) == 0
+    shim = ext.exl3_gemv_int8_max_k(0)
+    assert shim == 0
+    fused = {(u["int8_max_k"], u["K"], u["out_features"], u["mul1"]): u["fused"] for u in REF["use_mgemm"]}
     for K in range(1, 9):
-        assert ip.use_mgemm(K, 14336, mul1=True, device="cuda:0")          # gate/up: fused at every bitrate
-        assert ip.use_mgemm(K, 1024, mul1=True, device="cuda:0")           # k/v
-        assert ip.use_mgemm(K, 14336, mul1=False, device="cuda:0")         # other codebooks are always fused
-    monkeypatch.setattr(ext, "exl3_gemv_int8_max_k", lambda dev: 6)        # what the reference's own extension reports on sm_100
-    assert not ip.use_mgemm(4, 14336, mul1=True, device="cuda:0")          # wide 4 bpw pair: unfused there
-    assert ip.use_mgemm(4, 1024, mul1=True, device="cuda:0")               # narrow outputs stay fused either way
-    assert ip.use_mgemm(7, 14336, mul1=True, device="cuda:0")
+        assert fused[(shim, K, 14336, True)]                                # gate/up: fused at every bitrate
+        assert fused[(shim, K, 1024, True)]                                 # k/v
+        assert fused[(shim, K, 14336, False)]                               # other codebooks are always fused
+    assert not fused[(6, 4, 14336, True)]                                   # the reference's own extension on sm_100: wide 4 bpw pair unfused
+    assert fused[(6, 4, 1024, True)]                                        # narrow outputs stay fused either way
+    assert fused[(6, 7, 14336, True)]
 
 
-def test_reference_tp_import_split_equals_tp_slice(ref_exl3):
+def test_reference_tp_import_split_equals_tp_slice():
     """The reference's OWN shard construction (LinearEXL3.tp_export / tp_import_split, modules/quant/exl3.py:268-330), run with a
     trivial in-process stand-in for its SHM producer / consumer transport, against this repo's tp.tp_slice."""
-    ref_mod, _ = ref_exl3
     from exllamav3_b200 import tp
-
-    class Producer:
-        def send(self, t): return t
-
-    class Consumer:
-        def recv(self, t, cuda=False, slice_dim=None, first=None, last=None):
-            if t is None:
-                return None
-            return t if slice_dim is None else t.narrow(slice_dim, first, last - first).contiguous()
-
-    k, n = 512, 768
-    tens = _tensors(k, n)
-    g = torch.Generator().manual_seed(5)
-    tens["suh"] = torch.randn(k, generator=g).half(); tens["svh"] = torch.randn(n, generator=g).half()
-    bias = torch.randn(n, generator=g).half()
-    ref_full = ref_mod.LinearEXL3(None, k, n, bias=bias, out_dtype=torch.float, **tens)
+    ref = REF["tp_split"]
+    k, n, world = ref["k"], ref["n"], ref["world"]
+    tens, bias = refstubs.tp_tensors(k, n)
     mir_full = _qlin(tens, bias=bias, out_dtype=torch.float)
-    exported = ref_full.tp_export(None, Producer())
-    ctx = {"consumer": Consumer(), "device": "cpu"}
-    world = 3
     splits = [(True, a, b) for (a, b) in tp.split_ranges(n, world)] + [(False, a, b) for (a, b) in tp.split_ranges(k, world)] + [None]
-    for split in splits:
-        r = ref_mod.LinearEXL3.tp_import_split(ctx, exported, None, split)
+    assert [None if s is None else list(s) for s in splits] == [r["split"] for r in ref["splits"]]
+    for split, r in zip(splits, ref["splits"]):
         m = tp.tp_slice(mir_full, split)
-        assert (r.in_features, r.out_features, r.K, r.mcg, r.mul1, r.out_dtype) == (m.in_features, m.out_features, m.K, m.mcg, m.mul1, m.out_dtype)
-        assert torch.equal(r.trellis, m.trellis) and torch.equal(r.suh, m.suh) and torch.equal(r.svh, m.svh)
-        assert (r.bias is None) == (m.bias is None) and (r.bias is None or torch.equal(r.bias, m.bias))
+        assert (r["in_features"], r["out_features"], r["K"], r["mcg"], r["mul1"], DTYPES[r["out_dtype"]]) == \
+               (m.in_features, m.out_features, m.K, m.mcg, m.mul1, m.out_dtype)
+        for a in ("trellis", "suh", "svh", "bias"):
+            assert refstubs.digest(getattr(m, a)) == r[a], (split, a)
         assert m.trellis.is_contiguous()

@@ -206,6 +206,7 @@ def _two_rank_worker(rank, world, port, q):
         dist.destroy_process_group()
 
 
+@pytest.mark.gpu
 @pytest.mark.multigpu
 def test_fused_allreduce_two_gpus():
     if torch.cuda.device_count() < 2:
